@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU under torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port, all host threads), rank 0 only
+    python bench.py ... --dump-outputs DIR                   # also writes the PSM table of the last timed step as DIR/<field>.npy (dump_outputs)
 
 A "step" is one pass of the hot path over one batch of synthetic spectra. The headline workload is `cfg2` = BASELINE.json configs[1]:
 50k MS2 spectra x 200 peaks vs a ~2M-peptide tryptic index, +-20 ppm precursor / +-20 ppm fragment; per GPU the work is fixed (weak
@@ -29,6 +30,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -69,11 +71,15 @@ def spectra_per_rank(wl, world):
 
 
 def load_or_make(name, wl, rank, world):
-    """Synthetic peptide table (shared by all ranks; rank 0 generates and caches it under /tmp, the others wait for the file) and this rank's spectra."""
+    """Synthetic peptide table (shared by all ranks; rank 0 generates and caches it in the temporary directory, the others wait for the file) and
+    this rank's spectra. The cache belongs to this user and to the generator sources it was made by, so a table left by another user or by another
+    version of the generator is never read back."""
     from sage_b200 import Peptides, synth
     pk = dict(wl.get("peptides", {}))
-    tag = hashlib.sha1(json.dumps([wl["n_peptides"], sorted((k, str(v)) for k, v in pk.items())]).encode()).hexdigest()[:12]
-    cache = f"/tmp/sage_b200_pep_{tag}.npz"
+    h = hashlib.sha1(json.dumps([wl["n_peptides"], sorted((k, str(v)) for k, v in pk.items())]).encode())
+    for f in ("synth.py", os.path.join("csrc", "synth_expand.cpp")):
+        h.update(open(os.path.join(ROOT, "sage_b200", f), "rb").read())
+    cache = os.path.join(tempfile.gettempdir(), f"sage_b200_pep_{os.getuid()}_{h.hexdigest()[:12]}.npz")
     t0 = time.time()
     pep = None
     if rank != 0 and world > 1:
@@ -91,8 +97,13 @@ def load_or_make(name, wl, rank, world):
         pep = synth.make_peptides(wl["n_peptides"], **pk)
         if rank == 0:
             tmp = cache + f".{os.getpid()}.tmp.npz"
-            np.savez(tmp, **pep.__dict__)
-            os.replace(tmp, cache)
+            try:
+                np.savez(tmp, **pep.__dict__)
+                os.replace(tmp, cache)
+            except OSError as e:   # the cache only saves time: a full or read-only temporary directory does not stop the run
+                log(f"[rank 0] peptide table not cached ({e})")
+                if os.path.exists(tmp):
+                    os.unlink(tmp)
     spectra = synth.make_spectra(pep, spectra_per_rank(wl, world), seed=0xB200 + 2 + 1000 * rank, **wl["spectra"])
     log(f"[rank {rank}] {name} data: {len(pep)} peptides, {len(spectra)} spectra in {time.time() - t0:.1f}s")
     return pep, spectra
@@ -279,8 +290,35 @@ def base_config(name, wl, gpus, world):
             "l2": "per-step working set (index + ion tables >= 0.7 GB, spectra >= 40 MB) exceeds the 126 MB L2; no flush needed"}
 
 
-def run_workload(name, wl, steps, warmup, rank, local_rank, world, gpus, D, cpu, pageable=True):
-    """One workload on this repo's CUDA path. Returns the JSON-line dict (rank 0's view; all ranks must call it)."""
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, features, counts, report_psms):
+    """Writes a PSM table as the arrays a caller receives: <field>.npy for every Feature field, shape (spectra, report_psms), float32 for the f32
+    fields and float64 for the others (their integers are exact in it), and counts.npy. Rows past a spectrum's count are never written by the
+    library and are zeroed here. spectra.npy holds the spectrum indices the rows belong to: all of them, or a fixed seeded sample when the table
+    would exceed DUMP_BYTES."""
+    fields = [f for f in features.dtype.names if not f.startswith("_")]
+    n = len(counts)
+    feats = features.reshape(n, report_psms).copy()
+    feats[np.arange(report_psms)[None, :] >= np.asarray(counts)[:, None]] = np.zeros((), features.dtype)
+    per_spectrum = 16 + report_psms * sum(4 if features.dtype[f] == np.float32 else 8 for f in fields)
+    budget = DUMP_BYTES - 4096 * (len(fields) + 2)   # room for the .npy headers
+    idx = np.arange(n)
+    if n * per_spectrum > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n, budget // per_spectrum, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for f in fields:
+        a = feats[f][idx]
+        np.save(os.path.join(path, f"{f}.npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+    np.save(os.path.join(path, "counts.npy"), np.asarray(counts)[idx].astype(np.float64))
+    np.save(os.path.join(path, "spectra.npy"), idx.astype(np.float64))
+    log(f"outputs of the last timed step ({len(idx)} of {n} spectra) written to {path}")
+
+
+def run_workload(name, wl, steps, warmup, rank, local_rank, world, gpus, D, cpu, pageable=True, dump=None):
+    """One workload on this repo's CUDA path. Returns the JSON-line dict (rank 0's view; all ranks must call it). dump: directory that receives
+    rank 0's outputs of the last timed step of the resident path (dump_outputs)."""
     from sage_b200 import IndexedDatabase, Scorer, SpectraBatch, Tolerance, api
     pep, spectra = load_or_make(name, wl, rank, world)
     t0 = time.time()
@@ -331,6 +369,7 @@ def run_workload(name, wl, steps, warmup, rank, local_rank, world, gpus, D, cpu,
         D.barrier()
         wall_resident = time.perf_counter() - t0
         last = scorer.counters()
+        resident_out = scorer.download() if dump else None   # untimed: the last timed step's results, as a caller of run() receives them
         # ---- timed: K steps end to end through sage_b200_score_batch (pinned host in, pinned host out)
         D.barrier()
         t0 = time.perf_counter()
@@ -418,6 +457,8 @@ def run_workload(name, wl, steps, warmup, rank, local_rank, world, gpus, D, cpu,
                                     "tolerance": "every field bit-exact, incl. the f64 scores (device log == host libm log)" if f64_exact_default()
                                                  else "integer/f32 fields bit-exact; f64 scores rtol 1e-6 (tests/helpers.py)"}
         result["cpu_baseline"] = cpu_baseline_obj(rates, ns, threads)
+    if dump and rank == 0:
+        dump_outputs(dump, *resident_out, scorer.report_psms)
     del scorer, gdb
     for a in (hspec.masses, hspec.intensities, out, counts):
         api.pinned_free(a)
@@ -444,7 +485,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra workloads (cfg4 / cfg5 / cfg3) that follow the headline one")
     ap.add_argument("--extras", default="", help="comma-separated subset of the extra workloads to run")
     ap.add_argument("--spectra", type=int, default=0, help="override the number of spectra per GPU (profiling only; invalidates the metric)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the PSM table the last timed step of the headline workload computed (rank 0) as DIR/<name>.npy, "
+                         "at most 64 MB; the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "sage_b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl sage_b200)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -477,7 +525,8 @@ def main():
     # this rank's host thread (and the pinned buffers it is about to allocate) on the NUMA node next to its GPU
     node = api.bind_thread_to_device(local_rank)
     D = Dist(world, local_rank)
-    result = run_workload(args.workload, wl, args.steps, warmup, rank, local_rank, world, args.gpus, D, cpu=(args.gpus == 1 and not args.no_cpu_baseline))
+    result = run_workload(args.workload, wl, args.steps, warmup, rank, local_rank, world, args.gpus, D, cpu=(args.gpus == 1 and not args.no_cpu_baseline),
+                          dump=args.dump_outputs)
     result["numa_node"] = node
     extras = [] if (args.no_extras or args.spectra) else EXTRAS.get(args.workload, [])
     if args.extras:

@@ -10,21 +10,21 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = "/tmp/sage_b200_c_harness"
 
 
-def build_harness():
+def build_harness(out_dir):
     from sage_b200.build import build_library, library_path
     build_library()
     libdir = os.path.dirname(library_path())
+    exe = os.path.join(out_dir, "sage_b200_c_harness")
     subprocess.check_call(["/usr/bin/gcc", "-O2", "-Wall", "-I", os.path.join(ROOT, "include"), os.path.join(ROOT, "tests", "c_harness", "harness.c"),
-                           "-L", libdir, "-lsage_b200", f"-Wl,-rpath,{libdir}", "-o", EXE])
-    return EXE
+                           "-L", libdir, "-lsage_b200", f"-Wl,-rpath,{libdir}", "-o", exe])
+    return exe
 
 
-def test_harness_compiles_and_links_against_the_header():
+def test_harness_compiles_and_links_against_the_header(tmp_path):
     """CPU: the C program builds against include/sage_b200.h and resolves every symbol it uses from libsage_b200.so (no GPU call)."""
-    exe = build_harness()
+    exe = build_harness(tmp_path)
     out = subprocess.run(["ldd", exe], capture_output=True, text=True).stdout
     assert "libsage_b200.so" in out and "not found" not in out.split("libsage_b200.so")[1].splitlines()[0]
 
@@ -78,7 +78,7 @@ def read_output(path, report_psms):
 def test_c_harness_results_equal_the_oracle(tmp_path):
     from helpers import assert_features_equal, oracle_cfg, oracle_db_from_peptides
     from sage_b200 import Scorer, SpectraBatch, Tolerance, api, synth
-    exe = build_harness()
+    exe = build_harness(tmp_path)
     pep = synth.make_peptides(5000, seed=31, static_c=True)
     spectra = synth.make_spectra(pep, 900, seed=32)
     kw = dict(precursor_tol=Tolerance.ppm(-20, 20), fragment_tol=Tolerance.ppm(-10, 10), report_psms=2, min_isotope_err=-1, max_isotope_err=2, annotate_matches=True)

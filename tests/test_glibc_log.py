@@ -27,26 +27,26 @@ def log_inputs(n, seed):
     return np.concatenate(parts)
 
 
-def test_host_variant_matches_libm():
+def test_host_variant_matches_libm(tmp_path):
     """CPU: the variant the library selects equals this host's libm log() bit for bit on 3e6 inputs (the C++ evaluation is the same
     template the device compiles)."""
     from sage_b200 import api
     v = api.host_log_variant()
     assert v in (0, 1), "host libm is neither glibc log variant: f64 scores are only guaranteed to 1 ulp here"
     src = os.path.join(ROOT, "tests", "glibc_log_check.cpp")
-    exe = "/tmp/sage_b200_glibc_log_check"
+    exe = str(tmp_path / "sage_b200_glibc_log_check")
     subprocess.check_call(["g++", "-O2", "-I", os.path.join(ROOT, "sage_b200", "csrc"), src, "-o", exe])
     out = subprocess.check_output([exe, "3000000"]).decode()
     mism = dict(tok.split("=") for tok in out.split() if "=" in tok)
     assert int(mism["variant%d" % v]) == 0, out
 
 
-def test_host_log1pf_matches_libm_on_every_float():
+def test_host_log1pf_matches_libm_on_every_float(tmp_path):
     """CPU, exhaustive: the log1pf the kernels evaluate (OpenMS hyperscore, f32::ln_1p) equals this host's libm log1pf on all 2^32 floats."""
     from sage_b200 import api
     assert api.host_log1pf_exact()
     src = os.path.join(ROOT, "tests", "glibc_log1pf_check.cpp")
-    exe = "/tmp/sage_b200_glibc_log1pf_check"
+    exe = str(tmp_path / "sage_b200_glibc_log1pf_check")
     subprocess.check_call(["g++", "-O2", "-fopenmp", "-I", os.path.join(ROOT, "sage_b200", "csrc"), src, "-o", exe])
     out = subprocess.check_output([exe]).decode()
     assert "tested 4294967296 bad 0" in out, out

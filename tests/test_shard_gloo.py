@@ -2,6 +2,7 @@
 result identical (order and rebased spectrum indices) to a single-process run. The per-rank scorer here is the oracle —
 the sharding logic is independent of what scores a shard."""
 import os
+import socket
 import sys
 
 import numpy as np
@@ -41,8 +42,14 @@ def _worker(rank, world, port, tmp):
     dist.destroy_process_group()
 
 
+def _free_port():
+    with socket.socket() as s:   # a port the OS just handed out: on a shared host a fixed or pid-derived one may be taken
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
+
+
 def test_sharded_equals_single(tmp_path):
-    port = 29500 + (os.getpid() % 2000)
+    port = _free_port()
     mp.spawn(_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
     f, c = np.load(tmp_path / "f.npy"), np.load(tmp_path / "c.npy")
     f1, c1 = np.load(tmp_path / "f1.npy"), np.load(tmp_path / "c1.npy")
