@@ -237,6 +237,46 @@ int sage_b200_host_log1pf_exact(void);
 /* Test hook: out[i] = the device's evaluation of log(x[i]) with `variant` (0/1), or of (double)log1pf((float)x[i]) with variant 2 — compared bit for bit with the host libm by tests/test_glibc_log.py. */
 int sage_b200_device_log(int device, int variant, const double* x, uint64_t n, double* out);
 
+/* ---- Rescoring and FDR: the three steps the reference runs right after the search (runner.rs:533-537):
+ *   spectrum_fdr   LDA discriminant (linear_discriminant.rs:133-231), posterior error (kde.rs), sort, spectrum_q_value   runner.rs:280-291, qvalue.rs:8-36
+ *   picked_peptide / picked_protein   fdr.rs:16-190
+ * Strings never cross this boundary: the caller interns the reference's competition keys once per database (INTEGRATION.md). */
+typedef struct {
+    sage_b200_tolerance precursor_tol;  /* Scorer's precursor tolerance: Ppm or Da (Pct is rejected, as the reference's unreachable!) */
+    uint64_t n_peptides;                /* rows of the peptide table; when > 0 every Feature::peptide_idx must be below it (required with keys) */
+    const uint32_t* peptide_key;        /* [n_peptides] picked-peptide key per PeptideIx (fdr.rs:126-131); NULL skips picked_peptide */
+    uint64_t n_peptide_keys;            /* every peptide_key is < n_peptide_keys */
+    const uint32_t* protein_key;        /* [n_peptides] id of Peptide::proteins, UINT32_MAX when proteins.len() != 1 (fdr.rs:160-162); NULL skips picked_protein */
+    uint64_t n_protein_keys;            /* every other protein_key is < n_protein_keys */
+    const float* aligned_rt;            /* [n] Feature::aligned_rt (LDA feature 16); NULL = Feature::rt (scoring.rs:583) */
+    const float* delta_rt_model;        /* [n] Feature::delta_rt_model (feature 18); NULL = 0.999 (scoring.rs:584) */
+    const float* delta_ims_model;       /* [n] Feature::delta_ims_model (feature 19); NULL = 0.999 (scoring.rs:585) */
+} sage_b200_fdr_params;
+
+/* The Feature fields the three steps write, for features[i] (input order). peptide_q / protein_q stay 1.0 where that stage is skipped
+ * (and protein_q for peptides without a protein key); posterior_error stays 1.0 when the LDA cannot be fitted (scoring.rs:576-580). */
+typedef struct { float discriminant_score, posterior_error, spectrum_q, peptide_q, protein_q; } sage_b200_fdr_row;
+
+typedef struct {
+    uint64_t spectrum_passing, peptide_passing, protein_passing; /* the usize each step returns (q <= 0.01) */
+    double coef[20];                   /* LDA coefficients (NaN when not fitted) */
+    uint32_t lda_fitted;               /* 0: score_psms returned None and the heuristic score was used (runner.rs:284-287) */
+    float ms_h2d, ms_lda, ms_pep, ms_spectrum_q, ms_picked, ms_d2h; /* CUDA-event times of the phases, ms */
+    float ms_wall;                     /* host wall clock of the call, entry to return */
+} sage_b200_fdr_summary;
+
+/* Runs spectrum_fdr, picked_peptide and picked_protein over n Feature rows (any order: one score_batch result, or several concatenated).
+ * out[i] holds the fields for features[i]; order[r] (may be NULL) is the input index at rank r of the reference's sort (discriminant score
+ * descending, ties by input index), which a caller applies to its Vec<Feature>. summary may be NULL. n = 0 does nothing.
+ * Errors: EINVAL for a peptide_idx >= n_peptides, a key >= its count, keys without n_peptides, or a Pct tolerance; ELIMIT for n >= 2^32. */
+int sage_b200_assign_fdr(int device, const sage_b200_feature* features, uint64_t n, const sage_b200_fdr_params* params, sage_b200_fdr_row* out,
+                         uint32_t* order, sage_b200_fdr_summary* summary);
+
+/* LinearDiscriminantAnalysis::train (linear_discriminant.rs:63-124) on caller rows: rows is n x d row-major (d <= 20), decoy[i] != 0 for
+ * class 0. The same device reductions and host Gauss::solve as sage_b200_assign_fdr. Returns 0 with coef[0..d) written, 1 when the model
+ * cannot be fitted (an empty class, a failed solve or non-finite coefficients; coef is then NaN), or a negative error. */
+int sage_b200_lda_fit(int device, const double* rows, uint64_t n, uint32_t d, const uint8_t* decoy, double* coef);
+
 /* Page-locked host buffers: spectra/feature arrays placed here are copied by DMA without a staging memcpy. */
 void* sage_b200_host_alloc(size_t bytes);
 /* The same for a batch sage_b200_score_batch_multi cuts into n_devices contiguous blocks: the i-th of n equal parts of the buffer is placed on the

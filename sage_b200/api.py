@@ -89,6 +89,7 @@ EXPORTED_SYMBOLS = [
     "sage_b200_batch_download", "sage_b200_score_batch_multi", "sage_b200_quick_score", "sage_b200_initial_hits", "sage_b200_counters_get",
     "sage_b200_process_spectra", "sage_b200_find_reporter_ions", "sage_b200_host_alloc", "sage_b200_host_free", "sage_b200_last_error",
     "sage_b200_host_log_variant", "sage_b200_host_log1pf_exact", "sage_b200_device_log", "sage_b200_bind_thread_to_device", "sage_b200_host_alloc_blocks",
+    "sage_b200_assign_fdr", "sage_b200_lda_fit",
 ]
 
 _lib = None
@@ -583,6 +584,86 @@ def find_reporter_ions(peak_off, masses, intensities, labels, label_tolerance: T
     _check(load_library().sage_b200_find_reporter_ions(C.c_int(device), C.c_uint64(n), _ptr(peak_off), _ptr(masses), _ptr(intensities), _ptr(labels),
                                                        C.c_uint64(len(labels)), label_tolerance._c(), _ptr(out)))
     return out
+
+
+# ------------------------------------------------------------------------------------------------ rescoring + FDR
+class CFdrParams(C.Structure):
+    _fields_ = [("precursor_tol", CTol), ("n_peptides", C.c_uint64), ("peptide_key", C.c_void_p), ("n_peptide_keys", C.c_uint64),
+                ("protein_key", C.c_void_p), ("n_protein_keys", C.c_uint64), ("aligned_rt", C.c_void_p), ("delta_rt_model", C.c_void_p),
+                ("delta_ims_model", C.c_void_p)]
+
+
+FDR_SUMMARY_F32 = ["ms_h2d", "ms_lda", "ms_pep", "ms_spectrum_q", "ms_picked", "ms_d2h", "ms_wall"]
+
+
+class CFdrSummary(C.Structure):
+    _fields_ = [("spectrum_passing", C.c_uint64), ("peptide_passing", C.c_uint64), ("protein_passing", C.c_uint64), ("coef", C.c_double * 20),
+                ("lda_fitted", C.c_uint32)] + [(n, C.c_float) for n in FDR_SUMMARY_F32]
+
+
+# layout == sage_b200_fdr_row (include/sage_b200.h)
+FDR_DTYPE = np.dtype([("discriminant_score", "<f4"), ("posterior_error", "<f4"), ("spectrum_q", "<f4"), ("peptide_q", "<f4"), ("protein_q", "<f4")])
+
+
+def assign_fdr(features: np.ndarray, precursor_tol: Tolerance, peptide_key=None, protein_key=None, aligned_rt=None, delta_rt_model=None,
+               delta_ims_model=None, device: int = 0, *, n_peptides: int | None = None, n_peptide_keys: int | None = None, n_protein_keys: int | None = None):
+    """spectrum_fdr + picked_peptide + picked_protein (runner.rs:533-537) over Feature rows (FEATURE_DTYPE, any order).
+
+    peptide_key / protein_key: uint32 per PeptideIx (see include/sage_b200.h); None skips that stage. The key counts default to max + 1 and
+    n_peptides to the key table length. aligned_rt / delta_rt_model / delta_ims_model: optional float32 per feature (LDA features 16, 18, 19).
+    Returns (rows FDR_DTYPE[n] in input order, order uint32[n] = input index at each rank, summary dict)."""
+    f = np.ascontiguousarray(features)
+    if f.dtype != FEATURE_DTYPE:
+        raise TypeError("features must be FEATURE_DTYPE")
+    n = len(f)
+    keep: list = []
+
+    def arr(x, dt):
+        if x is None:
+            return None
+        a = np.ascontiguousarray(x, dtype=dt)
+        keep.append(a)
+        return a
+
+    pk, prk = arr(peptide_key, np.uint32), arr(protein_key, np.uint32)
+    p = CFdrParams()
+    p.precursor_tol = precursor_tol._c()
+    tables = [t for t in (pk, prk) if t is not None]
+    p.n_peptides = int(n_peptides if n_peptides is not None else (len(tables[0]) if tables else 0))
+    if pk is not None:
+        p.peptide_key = _ptr(pk)
+        p.n_peptide_keys = int(n_peptide_keys if n_peptide_keys is not None else (int(pk.max()) + 1 if len(pk) else 0))
+    if prk is not None:
+        p.protein_key = _ptr(prk)
+        valid = prk[prk != 0xFFFFFFFF]
+        p.n_protein_keys = int(n_protein_keys if n_protein_keys is not None else (int(valid.max()) + 1 if len(valid) else 0))
+    for name, x in (("aligned_rt", aligned_rt), ("delta_rt_model", delta_rt_model), ("delta_ims_model", delta_ims_model)):
+        a = arr(x, np.float32)
+        if a is not None and len(a) != n:
+            raise ValueError(f"{name} must have one value per feature")
+        setattr(p, name, _ptr(a))
+    rows = np.zeros(n, FDR_DTYPE)
+    order = np.zeros(n, np.uint32)
+    s = CFdrSummary()
+    _check(load_library().sage_b200_assign_fdr(C.c_int(device), _ptr(f), C.c_uint64(n), C.byref(p), _ptr(rows), _ptr(order), C.byref(s)))
+    summary = {k: getattr(s, k) for k, _ in CFdrSummary._fields_ if k != "coef"}
+    summary["coef"] = np.array(s.coef[:], np.float64)
+    summary["lda_fitted"] = bool(s.lda_fitted)
+    return rows, order, summary
+
+
+def lda_fit(rows: np.ndarray, decoy: np.ndarray, device: int = 0):
+    """LinearDiscriminantAnalysis::train (linear_discriminant.rs:63-124) on caller rows [n, d <= 20] through the device reductions:
+    the coefficients, or None when the model cannot be fitted."""
+    x = np.ascontiguousarray(rows, np.float64)
+    n, d = x.shape
+    dec = np.ascontiguousarray(decoy, np.uint8)
+    coef = np.zeros(d, np.float64)
+    rc = load_library().sage_b200_lda_fit(C.c_int(device), _ptr(x), C.c_uint64(n), C.c_uint32(d), _ptr(dec), _ptr(coef))
+    if rc == 1:
+        return None
+    _check(rc)
+    return coef
 
 
 Feature = FEATURE_DTYPE

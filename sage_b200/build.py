@@ -6,7 +6,7 @@ import subprocess
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 _SRC = os.path.join(_PKG, "csrc", "sage_b200.cu")
-_DEPS = [os.path.join(_PKG, "csrc", f) for f in ("sage_b200.cu", "kernels.cuh", "device_common.cuh")] + [
+_DEPS = [os.path.join(_PKG, "csrc", f) for f in ("sage_b200.cu", "kernels.cuh", "device_common.cuh", "fdr.cuh")] + [
     os.path.join(os.path.dirname(_PKG), "include", "sage_b200.h")]
 _OUT = os.path.join(_PKG, "lib", "libsage_b200.so")
 

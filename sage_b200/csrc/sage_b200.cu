@@ -200,6 +200,9 @@ static bool is_pinned(const void* p) {
     return a.type == cudaMemoryTypeHost;
 }
 
+// sage_b200_assign_fdr / sage_b200_lda_fit (uses fail, DevBuf, staged_h2d above)
+#include "fdr.cuh"
+
 // ------------------------------------------------------------------------------------------------ db
 struct BlockIndexSlot {
     WideIndexView v{};
