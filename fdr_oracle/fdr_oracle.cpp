@@ -7,8 +7,9 @@
 //   picked_peptide / protein crates/sage/src/fdr.rs:16-190 (Competition::assign_q_value :59-120)
 //
 // Test infrastructure only. Sums are sequential, as in the reference. Two things the reference leaves open are fixed here the way the device
-// library fixes them: the order among equal discriminant scores (par_sort_unstable_by) is ascending input index, and the competition rows,
-// which the reference collects from a hash map, start in key order (target before decoy) before the stable sort by score.
+// library fixes them: the order among equal discriminant scores (par_sort_unstable_by) is ascending input index, the competition rows,
+// which the reference collects from a hash map, start in key order (target before decoy) before the stable sort by score, and the per-key
+// maximum of +0 and -0 is +0 (max_total).
 // fo_set_block(B > 0) switches every f64 sum to blocks of B terms (a second summation order, used to measure how much the results move
 // under reordering; the reference's own KDE sums are rayon folds whose order changes from run to run).
 #include <omp.h>
@@ -282,6 +283,14 @@ uint64_t sort_spectrum_q(const float* disc, const uint8_t* decoy, uint64_t n, ui
     return passing;
 }
 
+// f32::max with NaN skipped; equal values of opposite sign (±0) are ordered as f32::total_cmp orders them, +0 above -0, so the result does
+// not depend on the order the features come in (the reference leaves that choice open; the device makes the same one)
+float max_total(float a, float b) {
+    if (std::isnan(b)) return a;
+    if (std::isnan(a)) return b;
+    return total_key(b) > total_key(a) ? b : a;
+}
+
 // fdr.rs:16-190 with integer keys: q per feature written to q (features without a key are left alone)
 uint64_t competition(const float* disc, const uint8_t* decoy, const uint32_t* key, uint64_t n, uint64_t n_keys, float* q) {
     const float lowest = -FLT_MAX;
@@ -290,8 +299,8 @@ uint64_t competition(const float* disc, const uint8_t* decoy, const uint32_t* ke
     for (uint64_t i = 0; i < n; i++) {
         const uint32_t k = key[i];
         if (k == 0xFFFFFFFFu) continue;
-        if (decoy[i]) { rev[k] = std::fmax(rev[k], disc[i]); has[k] |= 2; }
-        else { fwd[k] = std::fmax(fwd[k], disc[i]); has[k] |= 1; }
+        if (decoy[i]) { rev[k] = max_total(rev[k], disc[i]); has[k] |= 2; }
+        else { fwd[k] = max_total(fwd[k], disc[i]); has[k] |= 1; }
     }
     std::vector<double> scores;
     std::vector<uint8_t> is_decoy;
@@ -299,7 +308,7 @@ uint64_t competition(const float* disc, const uint8_t* decoy, const uint32_t* ke
     std::vector<Row> rows;
     for (uint64_t k = 0; k < n_keys; k++) {
         if (!has[k]) continue;
-        scores.push_back((double)std::fmax(fwd[k], rev[k]));
+        scores.push_back((double)max_total(fwd[k], rev[k]));
         is_decoy.push_back(rev[k] >= fwd[k]);
         if (has[k] & 1) rows.push_back({k, false, fwd[k], 1.0f});
         if (has[k] & 2) rows.push_back({k, true, rev[k], 1.0f});

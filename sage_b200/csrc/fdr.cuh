@@ -352,11 +352,20 @@ __global__ void k_posterior_error(const double* __restrict__ disc64, uint64_t n,
     }
 }
 
-// runner.rs:284-287: (-poisson as f32).ln_1p() + longest_y_pct / 3.0 in f32 (log1pf as glibc computes it); posterior_error keeps 1.0
+// runner.rs:284-287: (-poisson as f32).ln_1p() + longest_y_pct / 3.0 in f32 (log1pf as glibc computes it); posterior_error keeps 1.0.
+// NaN bits as the x86-64 host leaves them, where the device's own arithmetic would give its canonical 0x7fffffff: `-` flips a NaN's sign,
+// the f64 -> f32 conversion keeps the top 23 payload bits and quiets, `/` and `+` with one NaN operand return it quieted, an invalid `+`
+// (inf - inf) gives 0xffc00000, and when both addends are NaN the quotient's is returned (the host's operand order, pinned by a CPU test).
 __global__ void k_fallback(const sage_b200_feature* __restrict__ f, uint64_t n, float* __restrict__ disc32, float* __restrict__ pe) {
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
-        const float p = __double2float_rn(-f[i].poisson);
-        disc32[i] = __fadd_rn(glog::glibc_log1pf(p), __fdiv_rn(f[i].longest_y_pct, 3.0f));
+        const double poisson = f[i].poisson;
+        const uint64_t nb = (uint64_t)__double_as_longlong(poisson) ^ 0x8000000000000000ull;   // -poisson
+        const float p = isnan(poisson) ? __uint_as_float((uint32_t)(nb >> 32 & 0x80000000u) | 0x7fc00000u | (uint32_t)(nb >> 29 & 0x7fffffu))
+                                       : __double2float_rn(-poisson);
+        const float l = glog::glibc_log1pf(p), y = f[i].longest_y_pct;
+        const float q = isnan(y) ? __uint_as_float(__float_as_uint(y) | 0x00400000u) : __fdiv_rn(y, 3.0f);
+        const float s = __fadd_rn(l, q);
+        disc32[i] = isnan(q) ? q : isnan(l) ? l : isnan(s) ? __uint_as_float(0xffc00000u) : s;
         pe[i] = 1.0f;
     }
 }
@@ -419,7 +428,9 @@ __global__ void k_comp_init(uint64_t nk, uint32_t* __restrict__ fwd, uint32_t* _
     }
 }
 
-// fdr.rs:125-144 / 160-177: per key, forward / reverse = f32::max of the discriminant scores (NaN skipped), and which sides are present
+// fdr.rs:125-144 / 160-177: per key, forward / reverse = f32::max of the discriminant scores (NaN skipped), and which sides are present.
+// Equal values of opposite sign (±0) are ordered as f32::total_cmp orders them, +0 above -0, whatever order the features come in; the
+// reference's f32::max leaves that choice open, and fdr_oracle.cpp makes the same one.
 __global__ void k_comp_max(const sage_b200_feature* __restrict__ f, const float* __restrict__ disc32, uint64_t n, const uint32_t* __restrict__ key_of,
                            uint32_t* __restrict__ fwd, uint32_t* __restrict__ rev, uint32_t* __restrict__ flags) {
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
@@ -447,7 +458,7 @@ __global__ void k_comp_emit(const uint32_t* __restrict__ flags, const uint32_t* 
         const uint32_t fl = flags[k];
         if (!fl) continue;
         const float fw = from_total_key(fwd[k]), rv = from_total_key(rev[k]);
-        kx[key_pos[k]] = (double)fmaxf(fw, rv);
+        kx[key_pos[k]] = (double)from_total_key(max(fwd[k], rev[k]));   // in total order, as the per-side maxima: +0 above -0
         kdec[key_pos[k]] = rv >= fw;
         uint32_t p = row_pos[k];
         if (fl & 1u) { row_key[p] = fwd[k]; row_id[p] = (uint32_t)(2 * k); p++; }
@@ -920,7 +931,9 @@ extern "C" int sage_b200_assign_fdr(int device, const sage_b200_feature* feature
 
     // ---- validation, class counts, mass-error sample
     k_fdr_prep<<<grid_for(n), 256, 0, st>>>(B.f, n, is_da, npep, B.mass_err, B.dec, B.counters, B.err);
-    if (P->peptide_key || P->protein_key) k_check_keys<<<grid_for(npep), 256, 0, st>>>(B.pk, npk, B.prk, nprk, npep, B.err);
+    // a table the caller did not give has a zero-length slot, which aliases the next buffer: pass null for it
+    if (P->peptide_key || P->protein_key)
+        k_check_keys<<<grid_for(npep), 256, 0, st>>>(P->peptide_key ? B.pk : nullptr, npk, P->protein_key ? B.prk : nullptr, nprk, npep, B.err);
     CUDA_TRY(cudaGetLastError());
     unsigned long long n_decoy = 0;
     unsigned err = 0;

@@ -176,9 +176,10 @@ SB_HD float glibc_log1pf(float x) {
     int32_t k = 1, hu = 0;
     float f = 0.0f, c = 0.0f, u;
     if (hx < 0x3ed413d7) {                       // x < 0.41422
-        if (ax >= 0x3f800000) {                  // x <= -1.0
+        if (ax >= 0x3f800000) {                  // x <= -1.0, or a negative NaN
             if (x == -1.0f) return gf_flt((int32_t)0xff800000);   // log1p(-1) = -inf
-            return gf_flt(0x7fc00000);           // log1p(x < -1) = NaN (sign / payload not reproduced)
+            // (x - x) / (x - x) on x86-64 SSE: a NaN x comes back quieted, sign and payload kept; else the default NaN 0xffc00000
+            return gf_flt(ax > 0x7f800000 ? (hx | 0x00400000) : (int32_t)0xffc00000);
         }
         if (ax < 0x31000000) {                   // |x| < 2^-29
             if (ax < 0x24800000) return x;       // |x| < 2^-54
@@ -186,7 +187,8 @@ SB_HD float glibc_log1pf(float x) {
         }
         if (hx > 0 || hx <= (int32_t)0xbe95f61f) { k = 0; f = x; hu = 1; }   // -0.2929 < x < 0.41422
     }
-    if (hx >= 0x7f800000) return gf_add(x, x);
+    // x + x: +inf, or a NaN x quieted as the host leaves it (the device's own add would give its canonical 0x7fffffff)
+    if (hx >= 0x7f800000) return gf_flt(ax > 0x7f800000 ? (hx | 0x00400000) : hx);
     if (k != 0) {
         if (hx < 0x5a000000) {
             u = gf_add(1.0f, x);

@@ -14,7 +14,7 @@ int main() {
         volatile float vx = x;
         const float ref = log1pf(vx), got = sb::glog::glibc_log1pf(x);
         n++;
-        bad += memcmp(&ref, &got, 4) != 0 && !(ref != ref && got != got);
+        bad += memcmp(&ref, &got, 4) != 0;   // NaN results too: sign and payload as the host's SSE arithmetic leaves them
     }
     printf("tested %llu bad %llu\n", n, bad);
     return bad != 0;
